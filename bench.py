@@ -31,6 +31,10 @@ batch: tools/bench_cfg5.py runs config 5 over 1/2/4/8 GPUs through blance_ctx_cr
 
 --impl reference: the CPU arm — slices of the real workload's first inner plan through the
 literal oracle on the box's host cores (rank 0 only).
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed plan returned to its caller
+(blance_plan_fetch) as DIR/<name>.npy, so that two builds can be compared output for output on the same
+seeded cluster.
 """
 import argparse
 import json
@@ -165,6 +169,28 @@ def ncu_traffic(steps_per_launch):
         return None
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, res):
+    """next_rows / next_shape / warn of a PlanResult as float32 (node ids, shapes and warning flags are small
+    integers, exact in float32) and its counters (iters_run, converged, steps) as float64.  Above DUMP_LIMIT bytes
+    a fixed seeded sample of partitions is written, their indices in partition_index.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"next_rows": res.next_rows, "next_shape": res.next_shape, "warn": res.warn}
+    n_parts = res.next_rows.shape[0]
+    row_bytes = 4 * sum(a.shape[1] for a in arrays.values())
+    if n_parts * row_bytes > DUMP_LIMIT:
+        n_keep = (DUMP_LIMIT - 4096) // (row_bytes + 8)          # 4 KiB for the .npy headers and the counters
+        idx = np.sort(np.random.default_rng(0).choice(n_parts, n_keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        np.save(os.path.join(out_dir, "partition_index.npy"), idx.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+    np.save(os.path.join(out_dir, "counters.npy"), np.array([res.iters_run, res.converged, res.steps], np.float64))
+
+
 def shared_config(n_parts, n_nodes):
     """The part of `config` both arms print identically."""
     return {"workload": WORKLOAD if (n_parts, n_nodes) == (1048576, 1024) else
@@ -213,7 +239,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-string-api", action="store_true")
     ap.add_argument("--no-batch", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed plan's result arrays to DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs the GPU implementation: the reference arm times slices of a plan and returns no map")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -268,6 +298,8 @@ def main():
     barrier()
     launches = ctx.kernel_launches() - launches0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx.fetch(plan, tables.PlanResult(t)))
     total_ms = sum(kernel_ms)
     tt = torch.tensor([total_ms, sum(pass_ms)], dtype=torch.float64, device=dev)
     if dist is not None:
