@@ -290,11 +290,19 @@ __global__ void k_scatter_stream(DPool pool, int s, long long n_parts_total) {
     const uint32_t meta = (uint32_t)in[D.SLP];
     const int lo_s = D.state_slot_off[s], hi_s = D.state_slot_off[s + 1];
     // a step the speculative kernel accepted as sticky keeps its k current nodes, in (score, position) order:
-    // srank = 0x80 | rank of current node q in bits 2q..2q+1
+    // srank = 0x80 | rank of current node q in bits 2q..2q+1.  With k = 4 the flag shares bit 7 with the rank of the
+    // last node, so that rank is taken from the others: the ranks are a permutation of 0..k-1
     const uint32_t sr = pool.srank[g];
     int32_t sticky_out[4];
-    if (sr & 0x80u)
-      for (int q = 0; q < k && q < 4; ++q) sticky_out[(sr >> (2 * q)) & 3u] = in[lo_s + q];
+    if (sr & 0x80u) {
+      uint32_t rank_sum = 0;
+      for (int q = 0; q + 1 < k && q < 3; ++q) {
+        const uint32_t r = (sr >> (2 * q)) & 3u;
+        sticky_out[r] = in[lo_s + q];
+        rank_sum += r;
+      }
+      if (k >= 1 && k <= 4) sticky_out[(uint32_t)(k * (k - 1) / 2) - rank_sum] = in[lo_s + k - 1];
+    }
     const int32_t* out = (sr & 0x80u) ? sticky_out : out_rec;
     const int n_chosen = (sr & 0x80u) ? k : out_rec[k];
     int32_t* row = pool.rows + D.rows_off + (long long)p * D.SLP;

@@ -1059,16 +1059,19 @@ extern "C" int blance_moves_create(blance_ctx* ctx, int32_t n_parts, int32_t n_s
   cudaStream_t st = ctx->stream;
   const int max_ops = std::max(1, 2 * SL);
   const size_t P = (size_t)std::max(n_parts, 1), NN = (size_t)std::max(n_node_ids, 1);
-  size_t scan_tmp = 0, sort_tmp = 0;
+  // one temp buffer serves the scan of the op counts here, and the sort over partitions and the scan of the
+  // n_node_ids + 1 per-node counters in blance_moves_available
+  size_t scan_tmp = 0, sort_tmp = 0, node_scan_tmp = 0;
   cub::DeviceScan::ExclusiveSum(nullptr, scan_tmp, (const int32_t*)nullptr, (long long*)nullptr, n_parts + 1, st);
   cub::DeviceRadixSort::SortPairs(nullptr, sort_tmp, (const uint32_t*)nullptr, (uint32_t*)nullptr, (const int32_t*)nullptr, (int32_t*)nullptr, n_parts, 0, 32, st);
+  cub::DeviceScan::ExclusiveSum(nullptr, node_scan_tmp, (const int32_t*)nullptr, (int32_t*)nullptr, n_node_ids + 1, st);
   // scratch of the construction (rows, padded ops, counts) lives in the same arena and is simply left unused later
   struct Sl { void** p; size_t bytes; };
   blance_moves* mv = new blance_moves();
   mv->n_parts = n_parts; mv->n_node_ids = n_node_ids;
   int32_t *d_slot = nullptr, *d_beg = nullptr, *d_end = nullptr, *p_node = nullptr, *d_cnt = nullptr;
   uint8_t *p_state = nullptr, *p_kind = nullptr;
-  mv->tmp_bytes = std::max(scan_tmp, sort_tmp) + 256;
+  mv->tmp_bytes = std::max({scan_tmp, sort_tmp, node_scan_tmp}) + 256;
   std::vector<Sl> sl = {
       {(void**)&mv->d_off, sizeof(long long) * (P + 2)}, {(void**)&mv->d_node, sizeof(int32_t) * P * max_ops},
       {(void**)&mv->d_state, P * max_ops}, {(void**)&mv->d_kind, P * max_ops}, {(void**)&mv->d_next, sizeof(int32_t) * P},
